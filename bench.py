@@ -164,6 +164,17 @@ def build_workload(name, scale, state=True):
 AOS_SLOT = dict(stride=320, off_pos=32, off_v_and_m=16, off_dg_e=48, off_apic_b=96, col_pitch=16, off_vol=164)
 AOS_SCALAR = {scenes.MAT_LINEAR: -1, scenes.MAT_JELLY: -1, scenes.MAT_SNOW: 196, scenes.MAT_WATER: 204, scenes.MAT_SAND: 216}
 
+# --dump-outputs: particles written per run (120 bytes each: 31 MB for 262144) and the seed that picks them
+OUTPUT_SAMPLE = 262144
+OUTPUT_SEED = 20240917
+
+
+def dump_outputs(directory, arrays):
+    """One DIR/<name>.npy per array (float32 / float64)."""
+    os.makedirs(directory, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(directory, k + ".npy"), a)
+
 
 def slab_cuts(meta, res_z, world, weak):
     """Tile-layer cuts [(z0, z1)] * world by particle count: 1-D histogram of the base tile layer of the block's cell
@@ -369,8 +380,10 @@ class SlabJob:
         else:
             self.runner.substep(k)
 
-    def timed(self, steps, warmup, sample_clocks=True):
-        """W untimed + K timed substeps, barrier + synchronize on both sides, CUDA events, max over ranks."""
+    def timed(self, steps, warmup, sample_clocks=True, keep_outputs=False):
+        """W untimed + K timed substeps, barrier + synchronize on both sides, CUDA events, max over ranks.
+        keep_outputs: the particle state right after the K-th timed substep is kept in self.outputs (a sample, see
+        sample_outputs) before the per-stage pass below moves the scene on."""
         torch, e = self.torch, self.eng
         self.substep(warmup)
         self.barrier()
@@ -387,6 +400,8 @@ class SlabJob:
         clocks = sampler.stop() if sample_clocks else None
         ms_local = ev0.elapsed_time(ev1)
         c1 = e.get_counters()
+        if keep_outputs:
+            self.outputs = self.sample_outputs()
         # per-stage split: the same K substeps once more with CUDA events around every stage (untimed for `value`:
         # the event records cost a few microseconds per stage and switch the graph replay off)
         e.set_profiling(True)
@@ -410,6 +425,25 @@ class SlabJob:
         parts = [None] * self.world
         self.dist.all_gather_object(parts, mine)
         return {k: np.concatenate([p[k] for p in parts]) for k in keys} if self.rank == 0 else None
+
+    def sample_outputs(self, count=OUTPUT_SAMPLE):
+        """What mpmb_download_particles hands a caller, for a fixed seeded sample of particle ids (the whole set when it is
+        smaller), in id order, gathered on rank 0.  Particle ids are the seeding order, so two builds sample the same particles."""
+        keys = ("id", "x", "v", "F", "b", "mass", "vol", "ps", "group")
+        d = self.eng.download(sort_by_id=False)
+        if self.n_total > count:
+            want = np.sort(np.random.default_rng(OUTPUT_SEED).choice(self.n_total, count, replace=False))
+            keep = np.isin(d["id"], want)
+            d = {k: d[k][keep] for k in keys}
+        mine = {k: d[k] for k in keys}
+        if self.world > 1:
+            parts = [None] * self.world
+            self.dist.all_gather_object(parts, mine)
+            if self.rank != 0:
+                return None
+            mine = {k: np.concatenate([p[k] for p in parts]) for k in keys}
+        o = np.argsort(mine["id"], kind="stable")
+        return {k: mine[k][o].astype(np.float64 if k == "id" else np.float32) for k in keys}
 
     def close(self):
         self.eng.close()
@@ -517,12 +551,13 @@ def run_ours(args):
     job = SlabJob(args, cfg, rank, world, local, dist if world > 1 else None, weak=weak)
     n_total = job.n_total
     # ---- device-resident throughput, column at rest (the round-1 regime) ...
-    quiet = job.timed(args.steps, args.warmup)
+    dump = args.dump_outputs is not None
+    quiet = job.timed(args.steps, args.warmup, keep_outputs=dump and args.develop <= 0)
     # ---- ... and in a developed collapse: advance the same engine `develop` substeps, then time again
     flowing = None
     if args.develop > 0:
         job.substep(args.develop)
-        flowing = job.timed(args.steps, args.warmup)
+        flowing = job.timed(args.steps, args.warmup, keep_outputs=dump)
         flowing["developed_substeps"] = 2 * (args.warmup + args.steps) + args.steps + args.develop   # substeps behind the scene when its timed region starts
     head = quiet if (flowing is None or quiet["value"] <= flowing["value"]) else flowing
     head_name = "quiescent" if head is quiet else "flowing"
@@ -553,6 +588,8 @@ def run_ours(args):
             dist.barrier()
             dist.destroy_process_group()
         return
+    if dump:
+        dump_outputs(args.dump_outputs, job.outputs)
     peaks, peak_kind = measured_peaks()
     peak = float(peaks["hbm_gbs"])
     # dominant kernel of the (headline state's) substep on rank 0
@@ -698,7 +735,14 @@ def main():
     ap.add_argument("--migrate-capacity", type=int, default=65536, help="particles per face per substep (z-slab message size)")
     ap.add_argument("--exchange", default="peer", choices=["peer", "nccl"], help="z-slab transport: NVLink peer memory (default) or NCCL send/recv")
     ap.add_argument("--halo-capacity", type=int, default=0, help="active tiles per boundary layer (z-slab message size); 0 = the whole cross-section")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the particle state after the last timed substep as DIR/<field>.npy "
+                    "(a fixed seeded sample of %d particles, id order), for comparing two builds output for output" % OUTPUT_SAMPLE)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl == "reference":
+        # the CPU arm times a particle sample sized by a speed probe: its outputs are not the same particles from run to run
+        ap.error("--dump-outputs writes the GPU path's outputs; it does not apply to --impl reference")
     if args.develop < 0:
         args.develop = 20000 if args.workload == "sand256" else 2000
     if args.impl == "reference":

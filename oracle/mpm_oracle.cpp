@@ -1339,6 +1339,7 @@ void fast_substep(FastState &st, const Scene<float> &sc, Particles<float> &P, st
               _mm_store_ps(gn, _mm_add_ps(_mm_load_ps(gn), _mm_mul_ps(w, contrib)));
             }
       }
+      g_use_fast_svd = false;  // the switch is per thread: later svd3<float> calls on this thread take the checker path again
       tile_io(b, tile, true);
     }
   }
@@ -1427,6 +1428,7 @@ void fast_substep(FastState &st, const Scene<float> &sc, Particles<float> &P, st
       }
       if (bad) alive[i] = 0;
     }
+    g_use_fast_svd = false;
   }
   double t4 = now_s();
   st.t_sort += t1 - t0; st.t_p2g += t2 - t1; st.t_grid += t3 - t2; st.t_g2p += t4 - t3;

@@ -1,6 +1,7 @@
 """SURVEY §8f row 3: the AsyncMPM scheduler of the mirror (taichi_mpm_b200/async_mpm.py) against the REFERENCE's own AsyncMPM<3>
 object (src/async/async_mpm.{h,cpp} compiled in place, oracle/transfer_ref.cpp) — scheduler decisions identical (pool sizes,
-update counter, integer clock, time levels, survivors), particle states to fp32 rounding.  The substeps of the mirror run on a
+update counter, integer clock, time levels, survivors), particle states to fp32 rounding.  What the reference computed is
+committed (tests/golden/live_ref.npz, read through tests.common.live_ref).  The substeps of the mirror run on a
 stand-in engine here that executes the oracle's fp32 substep on the CPU (no GPU in this suite); tests/test_gpu_async.py runs the
 same comparison on the device engine."""
 import numpy as np
@@ -10,7 +11,6 @@ from oracle import pyoracle as O
 from taichi_mpm_b200 import async_mpm, capi, scenes
 from tests import common as T
 
-pytestmark = pytest.mark.skipif(not O.ref_transfer_available(), reason="reference build (oracle/_ref) not available")
 
 
 class OracleEngine:
@@ -49,13 +49,10 @@ class OracleEngine:
         pass
 
 
-def async_pair(kind, monkeypatch=None, engine_cls=None):
-    scene, st = T.perturbed_scene(kind, res=32, cells=8, seed=7, strain=0.0, vel=0.0, with_floor=False)
-    st["v"][:] = 0
-    st["v"][st["x"][:, 0] > 0.55, 0] = 10.0                    # a fast half: its blocks take a finer time level (cfl_dt_mul = 0.1)
-    unit = 2.5e-5 if kind == scenes.MAT_SNOW else 5e-6
-    kw = dict(unit_delta_t=unit, max_units=64, cfl_dt_mul=0.1)
-    ref = O.RefAsyncSolver(scene, st, **kw)
+def async_pair(kind, steps, monkeypatch=None, engine_cls=None):
+    """The scene, the reference's run of it (`steps` steps of AsyncMPM<3>, golden) and the mirror set up on the same state."""
+    scene, st, unit, kw = T.async_inputs(kind)
+    ref = T.live_ref("async_k%d_s%d" % (kind, steps))
     if engine_cls is not None:
         monkeypatch.setattr(capi, "Engine", engine_cls)
     m = async_mpm.AsyncMPM(res=(32, 32, 32), base_delta_t=unit, gravity=scene["gravity"], **kw)
@@ -66,27 +63,26 @@ def async_pair(kind, monkeypatch=None, engine_cls=None):
 
 
 def compare_async(ref, m, unit, steps, tol):
-    for _ in range(steps):
-        r = ref.step(80 * unit)
+    """ref: the reference's run (tests/golden/make_live_golden.py: async_ref): per-step decisions, survivors, a sample of particle states."""
+    assert len(ref["decisions"]) == steps
+    for r in ref["decisions"]:
         m.step(80 * unit)
         s = m.scheduler_stats()
-        assert (r["alive"], r["update_counter"], r["current_t_int"], r["min_level"], r["max_level"]) == \
-               (s["pool_entries"], s["update_counter"], s["current_t_int"], s["min_level"], s["max_level"])
+        assert tuple(int(v) for v in r) == (s["pool_entries"], s["update_counter"], s["current_t_int"], s["min_level"], s["max_level"])
     assert s["min_level"] < s["max_level"]                    # really asynchronous
-    pa, pm = ref.particles(), m.get_particles()
-    assert np.array_equal(np.nonzero(pa["alive"])[0], pm["id"])
-    ids = pm["id"]
-    assert np.abs(pa["x"][ids] - pm["x"]).max() <= tol["x"]
-    assert np.abs(pa["v"][ids] - pm["v"]).max() <= tol["v"] * np.abs(pa["v"]).max()
-    assert np.abs(pa["F"][ids] - pm["F"]).max() <= tol["F"]
-    assert m.update_counter == r["update_counter"] and m.num_particles() == len(ids)
+    pm = m.get_particles()
+    assert np.array_equal(ref["alive_ids"], pm["id"])
+    rows = np.searchsorted(pm["id"], ref["ids"])
+    assert np.abs(ref["x"] - pm["x"][rows]).max() <= tol["x"]
+    assert np.abs(ref["v"] - pm["v"][rows]).max() <= tol["v"] * float(ref["vmax"])
+    assert np.abs(ref["F"] - pm["F"][rows]).max() <= tol["F"]
+    assert m.update_counter == int(ref["decisions"][-1][1]) and m.num_particles() == len(pm["id"])
 
 
 @pytest.mark.parametrize("kind", [scenes.MAT_SNOW, scenes.MAT_SAND])
 def test_mirror_scheduler_makes_the_reference_s_decisions(kind, monkeypatch):
-    scene, st, unit, ref, m = async_pair(kind, monkeypatch, OracleEngine)
+    scene, st, unit, ref, m = async_pair(kind, 2, monkeypatch, OracleEngine)
     compare_async(ref, m, unit, steps=2, tol=dict(x=2e-6, v=2e-5, F=5e-5))
-    ref.close()
 
 
 def test_block_order_is_spgrid_s_and_types_without_a_limit_are_refused(monkeypatch):
@@ -102,27 +98,17 @@ def test_block_order_is_spgrid_s_and_types_without_a_limit_are_refused(monkeypat
 @pytest.mark.parametrize("kind", [scenes.MAT_SNOW, scenes.MAT_WATER, scenes.MAT_SAND, scenes.MAT_ELASTIC, scenes.MAT_VON_MISES, scenes.MAT_VISCO])
 def test_strength_limit_is_the_reference_particle_s_get_allowed_dt(kind):
     # the per-particle limit the scheduler reads (src/async/async_mpm.cpp:105-110) against the reference's own classes run in place
-    if not O.ref_particles_available():
-        pytest.skip("reference build (oracle/_ref) not available")
-    rng = np.random.default_rng(kind)
-    prm = scenes.material_params(kind)
-    n, dx = 40, 1.0 / 64
-    F = (np.eye(3)[None] + rng.normal(size=(n, 3, 3)) * 0.05).astype(np.float32)
-    ps = {scenes.MAT_SNOW: 1 + rng.normal(size=n) * 0.05, scenes.MAT_WATER: 1 + rng.normal(size=n) * 0.03}.get(kind, np.zeros(n)).astype(np.float32)
-    v = rng.normal(size=(n, 3)).astype(np.float32) * 2
-    vol = np.full(n, dx ** 3 / 8, np.float32)
-    mass = vol * np.float32(400.0)
-    Fcm = np.ascontiguousarray(np.transpose(F, (0, 2, 1)).reshape(n, 9))       # column-major, as the engine and the oracle carry it
-    got = async_mpm.allowed_dt(kind, prm, F.reshape(n, 9), ps, mass, vol, v, dx)   # the determinant does not care about the layout
-    ref = np.array([O.ref_allowed_dt(kind, prm, Fcm[i], float(ps[i]), float(mass[i]), float(vol[i]), v[i], dx) for i in range(n)])
+    # (golden: tests/golden/make_live_golden.py strength_ref, which hands the reference F column-major, as the engine and the oracle carry it)
+    F, ps, v, vol, mass, dx = T.strength_inputs(kind)
+    got = async_mpm.allowed_dt(kind, scenes.material_params(kind), F.reshape(len(F), 9), ps, mass, vol, v, dx)   # the determinant does not care about the layout
+    ref = T.live_ref("allowed_dt")["k%d" % kind]
     assert np.abs(got - ref).max() <= 2e-6 * ref.max()
 
 
 def test_types_without_a_strength_limit_return_zero_in_the_reference_too():
-    if not O.ref_particles_available():
-        pytest.skip("reference build (oracle/_ref) not available")
+    ref = T.live_ref("allowed_dt")
     for kind in (scenes.MAT_LINEAR, scenes.MAT_JELLY):
-        assert O.ref_allowed_dt(kind, scenes.material_params(kind), np.eye(3).reshape(9), 0.0, 1e-3, 1e-6, np.zeros(3), 1 / 64) == 0.0
+        assert ref["k%d" % kind] == 0.0
         with pytest.raises(ValueError):
             async_mpm.allowed_dt(kind, scenes.material_params(kind), np.eye(3, dtype=np.float32).reshape(1, 9), np.zeros(1, np.float32),
                                  np.ones(1, np.float32), np.ones(1, np.float32), np.zeros((1, 3), np.float32), 1 / 64)
@@ -148,7 +134,6 @@ def test_async_mirror_frame_dump_comes_from_the_pools(monkeypatch, tmp_path):
 def test_mirror_scheduler_follows_the_reference_through_deletions_and_level_changes(monkeypatch):
     # eight steps: the fast half of the block runs into the deletion band (4096 -> 3874 pool entries), levels regroup every step;
     # the two schedulers stay in lockstep (≈ 400 000 particle updates)
-    scene, st, unit, ref, m = async_pair(scenes.MAT_SNOW, monkeypatch, OracleEngine)
+    scene, st, unit, ref, m = async_pair(scenes.MAT_SNOW, 8, monkeypatch, OracleEngine)
     compare_async(ref, m, unit, steps=8, tol=dict(x=5e-6, v=1e-4, F=2e-4))
     assert m.scheduler_stats()["pool_entries"] < 3900
-    ref.close()

@@ -1,21 +1,27 @@
 """Frame output (SURVEY §8f row 1): the product's BGEO writer against the reference's own writer.
 
 Golden files under tests/golden/ were written by the Partio copy vendored in the reference tree
-(tests/golden/make_bgeo_golden.py); where that tree is present (the build container) the writer is
-also compared live, including the 65536-point switch of the primitive's index width."""
+(tests/golden/make_bgeo_golden.py); larger files of that writer, including the 65536-point switch of the primitive's
+index width, and a frame of the reference solver's write_partio are pinned by size and SHA-256 (tests/golden/live_ref.npz,
+tests/golden/make_live_golden.py)."""
+import hashlib
 import importlib.util
 import os
 
 import numpy as np
 import pytest
 
-from oracle import pyoracle as O
 from taichi_mpm_b200 import bgeo, mpm
+from tests import common as T
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 _spec = importlib.util.spec_from_file_location("make_bgeo_golden", os.path.join(HERE, "golden", "make_bgeo_golden.py"))
 G = importlib.util.module_from_spec(_spec)
 _spec.loader.exec_module(G)
+
+
+def _same_file(data, ref):
+    assert len(data) == int(ref["size"]) and hashlib.sha256(data).digest() == ref["sha256"].tobytes()
 
 
 @pytest.mark.parametrize("name,n,seed,verbose", [("frame_plain_17", 17, 1, False), ("frame_verbose_9", 9, 2, True), ("frame_empty", 0, 3, False)])
@@ -44,40 +50,28 @@ def test_reader_round_trip_of_reference_file():
     assert np.array_equal(d["debug"][water, 0], p["ps"][water]) and not d["debug"][~water, 0].any()
 
 
-@pytest.mark.skipif(not O.partio_ref_available(), reason="reference tree absent: golden files only")
-@pytest.mark.parametrize("n,verbose", [(1, False), (65536, False), (65537, False), (70001, True)])
+@pytest.mark.parametrize("n,verbose", T.BGEO_CASES)
 def test_writer_equals_reference_writer_live(tmp_path, n, verbose):
     p = G.golden_particles(n, 40 + n % 7)
     attrs = mpm.frame_attributes(p, G.GROUP_KINDS, verbose)
-    mine, ref = tmp_path / "mine.bgeo", tmp_path / "ref.bgeo"
+    mine = tmp_path / "mine.bgeo"
     bgeo.write_bgeo(str(mine), p["x"], attrs)
-    d = {a[0]: a[2] for a in attrs}
-    vb = {k: d[k] for k in ("m", "boundary_normal", "debug", "states", "boundary_distance", "near_boundary", "apic_frobenius_norm")} if verbose else None
-    O.ref_write_partio(str(ref), p["x"], d["v"], d["type"], d["index"], d["limit"], vb)
-    assert mine.read_bytes() == ref.read_bytes()
+    _same_file(mine.read_bytes(), T.live_ref("bgeo_n%d_v%d" % (n, verbose)))     # make_live_golden.py: bgeo_writer_ref
 
 
-@pytest.mark.skipif(not O.ref_transfer_available(), reason="reference tree absent")
 def test_writer_equals_write_partio_of_the_reference_solver_live(tmp_path):
     # the reference's MPM<3> (oracle/transfer_ref.cpp) steps a scene, deletes a particle, and dumps the frame with
-    # its own write_partio; the product's writer, given the same particle state, produces the same bytes
-    from tests import common as T
+    # its own write_partio (make_live_golden.write_partio_ref); the product's writer, given the same particle state,
+    # produces the same bytes
     from taichi_mpm_b200 import scenes
-    scene, st = T.perturbed_scene(scenes.MAT_SAND, res=24, cells=3, seed=2)
-    st["x"][0] = [6.5 / 24, 0.5, 0.5]
-    s = O.RefSolver(scene, st)
-    alive = s.substep(5)
-    ref = tmp_path / "ref.bgeo"
-    s.write_partio(ref)
-    p = s.particles()
-    s.close()
-    ids = p["alive_ids"]
-    assert alive == len(ids) == len(st["x"]) - 1
-    d = dict(id=ids.astype(np.uint32), x=p["x"][ids], v=p["v"][ids], b=p["b"][ids], mass=st["mass"][ids], ps=p["ps"][ids],
-             group=np.zeros(len(ids), np.int32))
+    scene, st = T.write_partio_scene()
+    p = T.live_ref("write_partio")
+    ids = p["ids"]
+    assert int(p["alive"]) == len(ids) == len(st["x"]) - 1
+    d = dict(id=ids.astype(np.uint32), x=p["x"], v=p["v"], b=p["b"], mass=st["mass"][ids], ps=p["ps"], group=np.zeros(len(ids), np.int32))
     mine = tmp_path / "mine.bgeo"
     bgeo.write_bgeo(str(mine), d["x"], mpm.frame_attributes(d, [scenes.MAT_SAND], verbose=False))
-    assert mine.read_bytes() == ref.read_bytes()
+    _same_file(mine.read_bytes(), p)
 
 
 def test_read_rejects_other_files(tmp_path):

@@ -78,16 +78,10 @@ def test_same_script_on_the_mirror_and_on_the_reference_solver():
     solver, add_particles, step) run (a) on the reference's OWN MPM<3> object — its add_particles(benchmark=125), its
     substep(), compiled in place for the CPU (oracle/transfer_ref.cpp) — and (b) on the mirror MPM driving the CUDA
     engine through the C-ABI.  Same particles, same motion."""
-    from oracle import pyoracle as O
-    if not O.ref_transfer_available():
-        pytest.skip("reference build (oracle/_ref) not available")
     from taichi_mpm_b200 import MPM, scenes
-    res, dt, nsub = 40, 1e-4, 20
-    ref = O.RefSolver.from_benchmark(res, dt, (0.0, -10.0, 0.0), "jelly", benchmark=125, density=400.0)
-    n = ref.n
-    ref.substep(nsub)
-    r = ref.particles()
-    ref.close()
+    r = T.live_ref("bench_script")                                             # the reference's run (tests/golden/make_live_golden.py)
+    res, dt, nsub = T.BENCH_SCRIPT["res"], T.BENCH_SCRIPT["dt"], T.BENCH_SCRIPT["nsub"]
+    n = int(r["n"])
     lo = int(round(res * 0.4)); hi = lo + int(round(res * 0.2))
     x0, _, _ = scenes.lattice_block(res, (lo,) * 3, (hi,) * 3, 400.0, 0.0)
     m = MPM(res=(res, res, res), base_delta_t=dt, gravity=(0, -10, 0))
@@ -96,10 +90,11 @@ def test_same_script_on_the_mirror_and_on_the_reference_solver():
     for _ in range(nsub):
         m.step(-1.0)                                                           # dt < 0: exactly one substep
     p = m.get_particles()
-    assert np.array_equal(p["id"], np.arange(n, dtype=p["id"].dtype)) and len(r["alive_ids"]) == n
-    assert np.abs(p["x"] - r["x"]).max() <= 1e-5
-    assert np.abs(p["v"] - r["v"]).max() <= 1e-3 * np.abs(r["v"]).max()
-    assert np.abs(p["F"] - r["F"]).max() <= 2e-4
+    assert np.array_equal(p["id"], np.arange(n, dtype=p["id"].dtype)) and int(r["alive"]) == n
+    ids = r["ids"]
+    assert np.abs(p["x"][ids] - r["x"]).max() <= 1e-5
+    assert np.abs(p["v"][ids] - r["v"]).max() <= 1e-3 * float(r["vmax"])
+    assert np.abs(p["F"][ids] - r["F"]).max() <= 2e-4
 
 
 def test_reference_solver_object_steps_through_libmpmb(tmp_path):

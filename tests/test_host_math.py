@@ -13,6 +13,7 @@ import pytest
 
 from oracle import pyoracle as O
 from taichi_mpm_b200 import scenes
+from tests import common as T
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _SRC = os.path.join(_HERE, "host_math", "host_math.cpp")
@@ -38,11 +39,7 @@ def _p(a):
     return a.ctypes.data_as(C.c_void_p)
 
 
-def _params8(kind, **kw):
-    p = np.zeros(8, np.float32)
-    q = scenes.material_params(kind, **kw)
-    p[: min(8, len(q))] = q[:8]
-    return p
+_params8 = T.params8
 
 
 def _cm(M):
@@ -156,26 +153,19 @@ def test_device_sand_large_strain_matches_oracle_for_non_inverted_elements(hm):
     assert np.abs(_math(force) - fo)[ok].max() <= 2e-4 * np.abs(fo[ok]).max()
 
 
-@pytest.mark.skipif(not O.ref_particles_available(), reason="reference tree absent")
 @pytest.mark.parametrize("kind,strain,rate", [(scenes.MAT_LINEAR, 0.05, 0.01), (scenes.MAT_JELLY, 0.1, 0.01), (scenes.MAT_SNOW, 0.03, 0.01),
                                               (scenes.MAT_WATER, 0.0, 0.01), (scenes.MAT_SAND, 2e-3, 1e-3), (scenes.MAT_SAND, 0.05, 0.02),
                                               (scenes.MAT_ELASTIC, 0.05, 0.01), (scenes.MAT_VON_MISES, 0.02, 0.01), (scenes.MAT_VISCO, 0.05, 0.01)])
 def test_device_material_step_matches_reference_particles_directly(hm, kind, strain, rate):
     # the CUDA header's fused step against the REFERENCE's own plasticity() + calculate_force()
-    # (src/particles.cpp compiled in place with the stand-in core, oracle/particles_ref.cpp): no oracle in between
-    rng = np.random.default_rng(50 + kind)
+    # (src/particles.cpp compiled in place with the stand-in core, oracle/particles_ref.cpp): no oracle in between;
+    # what the reference computed is committed (tests/golden/make_live_golden.py: material_ref)
+    ref = T.live_ref("material_c%d" % T.MATERIAL_CASES.index((kind, strain, rate)))
     prm = _params8(kind)
-    n, vol = 120, np.float32(1e-6)
+    vol = np.float32(T.MATERIAL_VOL)
     worst_F = worst_ps = worst_f = scale = 0.0
-    for _ in range(n):
-        F = (np.eye(3) + rng.normal(size=(3, 3)) * strain).astype(np.float32)
-        cdg = (np.eye(3) + rng.normal(size=(3, 3)) * rate).astype(np.float32)
-        if np.linalg.det(F.astype(np.float64)) < 0.3:
-            continue
-        ps = np.float32({scenes.MAT_SNOW: 1 + rng.normal() * 0.05, scenes.MAT_WATER: 1 + rng.normal() * 0.02,
-                         scenes.MAT_SAND: abs(rng.normal()) * 2e-3 * (rng.random() < 0.5),
-                         scenes.MAT_VISCO: 1000.0 * (0.5 + rng.random())}.get(kind, 0.0))
-        Fr, psr, fr = O.ref_particle_step(kind, prm, cdg, F, ps, float(vol))
+    for i, (F, cdg, ps) in enumerate(T.material_states(kind, strain, rate)):
+        Fr, psr, fr = ref["F"][i], float(ref["ps"][i]), ref["force"][i]
         Fd, psd, force = _cm(F[None]), np.array([ps], np.float32), np.zeros((1, 9), np.float32)
         hm.hm_material_step(C.c_int64(1), C.c_int(kind), _p(prm), _p(_cm(cdg[None])), _p(Fd), _p(psd), _p(np.array([vol], np.float32)), _p(force))
         if kind != scenes.MAT_WATER:

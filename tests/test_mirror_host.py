@@ -213,13 +213,11 @@ def test_step_counts_match_the_reference_step_golden(monkeypatch):
 
 
 def test_step_counts_match_the_reference_step_live(monkeypatch):
-    from oracle import pyoracle as O
-    if not O.ref_transfer_available():
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
-    from tests.golden import make_step_golden as G
-    want, cur, req = G.reference_counts(2e-5, 0.004, 25)
-    got, m = _mirror_counts(monkeypatch, 2e-5, 0.004, 25)
-    assert np.array_equal(got, want) and m.current_t == cur and m.request_t == req
+    # a frame length that is not a multiple of the substep (tests/golden/make_live_golden.py: step_ref)
+    from tests import common as T
+    ref = T.live_ref("step")
+    got, m = _mirror_counts(monkeypatch, *T.STEP_LIVE)
+    assert np.array_equal(got, ref["counts"]) and m.current_t == ref["clocks"][0] and m.request_t == ref["clocks"][1]
 
 
 def test_add_particles_follows_the_reference_rules(fake_engine):

@@ -77,10 +77,10 @@ def test_oracle_constitutive_matches_reference_particles_live(kind):
         assert np.abs(O.calculate_force(kind, prm.astype(np.float64), F.astype(np.float64), float(ps), G.VOL, np.float64) - f0).max() <= FORCE_TOL[kind] * max(np.abs(f0).max(), scale)
 
 
-@pytest.mark.skipif(not O.ref_particles_available(), reason="reference tree absent")
 def test_sand_alpha_and_defaults_live():
-    L = O.ref_particles()
-    for phi in (10.0, 30.0, 45.0):
-        assert abs(L.ref_sand_alpha(O.C.c_float(phi)) - scenes.material_params(scenes.MAT_SAND, friction_angle=phi)[2]) <= 1e-7
+    from tests import common as T
+    ref = T.live_ref("sand")                  # the reference's own values (tests/golden/make_live_golden.py sand_ref)
+    for alpha, phi in zip(ref["alpha"], (10.0, 30.0, 45.0)):
+        assert abs(alpha - scenes.material_params(scenes.MAT_SAND, friction_angle=phi)[2]) <= 1e-7
     for kind in range(5):
-        assert np.allclose(O.ref_default_params(kind), scenes.material_params(kind), rtol=3e-7, atol=0)
+        assert np.allclose(ref["defaults"][kind], scenes.material_params(kind), rtol=3e-7, atol=0)

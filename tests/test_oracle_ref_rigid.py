@@ -75,23 +75,14 @@ def test_oracle_cpic_matches_reference_live(variant):
     _compare(scene, st, rigid, ref)
 
 
-@pytest.mark.skipif(not O.ref_transfer_available(), reason="reference build (oracle/_ref) not available")
 def test_rigid_pages_are_the_reference_s_including_its_one_sided_dilation():
     # update_rigid_page_map tests the OFFSET of the neighbour loop against [0, spgrid_size) (src/mpm.cpp:1062), so a block with a
     # rigid particle flags itself and its upper neighbours only; the restatement follows that, and so does the engine
+    # (the pages the reference flags in the scanned window are stored: tests/golden/make_live_golden.py rigid_pages_ref)
     scene, st, rigid = G.golden_scene("kinematic")
-    s = O.RefSolver(scene, st)
-    s.set_rigid(rigid)
-    s.coupled_stage(0)
     pos = rigid["position"][rigid["sample_rigid"]] + rigid["sample_offset"] @ rigid["rot"][1].reshape(3, 3).T.T   # world anchors (one body)
     base = (pos * scene["res"][0] - 0.5).astype(int)
     blocks = {(b[0] >> 2, b[1] >> 2, b[2] >> 3) for b in base}
     expect = {(x + i, y + j, z + k) for (x, y, z) in blocks for i in (0, 1) for j in (0, 1) for k in (0, 1)}
-    got = set()
-    for x in range(0, 9):
-        for y in range(0, 9):
-            for z in range(0, 5):
-                if s.is_rigid_page((4 * x, 4 * y, 8 * z)):
-                    got.add((x, y, z))
-    s.close()
+    got = {tuple(int(c) for c in p) for p in T.live_ref("rigid_pages")["kinematic"]}
     assert got == expect and any((x - 1, y, z) not in got for (x, y, z) in blocks)

@@ -32,8 +32,11 @@ _spec.loader.exec_module(G)
 TOL = dict(grid=3e-6, x=2e-7, v=3e-6, F=2e-6, b=4e-5, ps=1e-5)
 
 
-def _compare(scene, st, grid_ref, p_ref):
+def _compare(scene, st, grid_ref, p_ref, rows=None):
+    """rows: the particles p_ref holds (all when None)."""
     new, grid_rast, _ = O.substep(scene, st, np.float64)
+    if rows is not None:
+        new = {k: a[rows] for k, a in new.items()}
     pmax = max(np.abs(grid_rast[..., :3]).max(), grid_rast[..., 3].max())
     assert np.abs(grid_ref - grid_rast).max() <= TOL["grid"] * pmax
     assert (grid_ref[..., 3] > 0).sum() == (grid_rast[..., 3] > 0).sum()             # the same set of touched nodes
@@ -132,36 +135,22 @@ def test_timed_cpu_port_matches_golden_run_of_reference_substep(kind):
     assert T.ps_err(f.st["ps"][ids], ref["ps"]) <= (5e-4 if kind == scenes.MAT_VISCO else 5e-5)
 
 
-@pytest.mark.skipif(not O.ref_transfer_available(), reason="reference tree absent")
 def test_two_materials_in_one_scene_match_reference_substep_live():
     # sand resting next to water, each with its own registered particle type in the reference's allocator
-    res = 32
-    xa, ma, va = scenes.lattice_block(res, (10, 10, 10), (15, 15, 15), 400.0, 0.05)
-    xb, mb, vb = scenes.lattice_block(res, (15, 10, 10), (19, 14, 14), 400.0, 0.05, seed=5)
-    sa = scenes.make_state(xa, ma, va, scenes.MAT_SAND, 0)
-    sb = scenes.make_state(xb, mb, vb, scenes.MAT_WATER, 1)
-    st = {k: np.concatenate([sa[k], sb[k]]) for k in sa}
-    rng = np.random.default_rng(12)
-    st["v"] = (rng.normal(size=st["x"].shape) * 0.3).astype(np.float32)
-    planes = np.array([[0, 1, 0, -10.4]], np.float32)
-    scene = dict(res=(res,) * 3, dx=1.0 / res, dt=2e-5, gravity=(0.0, -10.0, 0.0), particle_gravity=1,
-                 mat_kind=np.array([scenes.MAT_SAND, scenes.MAT_WATER], np.int32),
-                 mat_params=np.stack([scenes.material_params(scenes.MAT_SAND), scenes.material_params(scenes.MAT_WATER)]),
-                 planes=planes, sdf=scenes.planes_sdf(res, planes), friction=0.4)
-    s = O.RefSolver(scene, st)
-    alive = s.substep(15)
-    p = s.particles()
-    s.close()
+    # (tests/common.py: two_materials_scene; the reference's 15 substeps are stored, a seeded sample of the particles)
+    scene, st = T.two_materials_scene()
+    p = T.live_ref("two_materials")
     cur = st
     for _ in range(15):
         cur, _, _ = O.substep(scene, cur, np.float64)
     ids = np.nonzero(cur["alive"])[0]
-    assert alive == len(ids) == len(st["x"]) and np.array_equal(p["alive_ids"], ids)
-    assert np.abs(p["x"] - cur["x"]).max() <= TOL_SUB["x"]
-    assert np.abs(p["v"] - cur["v"]).max() <= TOL_SUB["v"] * np.abs(cur["v"]).max()
-    sand = st["group"] == 0
-    assert np.abs(p["F"][sand] - cur["F"][sand]).max() <= TOL_SUB["F"]
-    assert T.ps_err(p["ps"], cur["ps"]) <= TOL_SUB["ps"]
+    assert int(p["alive"]) == len(ids) == len(st["x"]) and np.array_equal(p["alive_ids"], ids)
+    s = p["ids"]
+    assert np.abs(p["x"] - cur["x"][s]).max() <= TOL_SUB["x"]
+    assert np.abs(p["v"] - cur["v"][s]).max() <= TOL_SUB["v"] * np.abs(cur["v"]).max()
+    sand = st["group"][s] == 0
+    assert np.abs(p["F"][sand] - cur["F"][s][sand]).max() <= TOL_SUB["F"]
+    assert T.ps_err(p["ps"], cur["ps"][s]) <= TOL_SUB["ps"]
 
 
 @pytest.mark.skipif(not O.ref_transfer_available(), reason="reference tree absent: golden vectors only")
@@ -189,49 +178,45 @@ def test_oracle_transfers_match_reference_loops_live(kind):
         _compare(scene, st, grid, p)
 
 
-@pytest.mark.skipif(not O.ref_transfer_available(), reason="reference tree absent")
 @pytest.mark.parametrize("friction", [-1.0, -2.0, -2.3, 0.0, 0.4, 5.0])
 @pytest.mark.parametrize("particle_gravity", [1, 0])
 def test_grid_update_modes_match_reference_live(friction, particle_gravity):
     # sticky (-1), slip (<= -2, with friction -mu-2), separate with Coulomb friction (>= 0): src/mpm_fwd.h:25-57 as
     # apply_grid_boundary_conditions uses it (src/mpm.cpp:296-372); gravity on the grid when particle_gravity is
-    # off (src/mpm.cpp:519-527)
-    from tests import common as T
-    scene, st = T.perturbed_scene(scenes.MAT_JELLY, res=24, cells=4, seed=41, friction=friction)
-    scene["particle_gravity"] = particle_gravity
+    # off (src/mpm.cpp:519-527).  The reference's node velocities after its own P2G + grid update are stored.
+    scene, st = T.grid_update_scene(friction, particle_gravity)
     _, grid_rast, grid_vel = O.substep(scene, st, np.float64)
-    s = O.RefSolver(scene, st)
-    s.p2g(True)
-    s.grid_update()
-    g = s.get_grid()
-    s.close()
+    r = T.live_ref("grid_update_f%g_g%d" % (friction, particle_gravity))
+    g = np.zeros((grid_rast[..., 0].size, 3), np.float32)
+    g[r["idx"]] = r["vel"]
+    g = g.reshape(grid_rast.shape[:3] + (3,))
     act = grid_rast[..., 3] > 0
-    assert np.abs(g[..., :3] - grid_vel[..., :3])[act].max() <= 5e-6 * np.abs(grid_vel[..., :3]).max()
+    assert np.abs(g - grid_vel[..., :3])[act].max() <= 5e-6 * np.abs(grid_vel[..., :3]).max()
 
 
-@pytest.mark.skipif(not O.ref_transfer_available(), reason="reference tree absent")
 def test_lattice_generator_matches_reference_benchmark_seeding_live():
     # the synthetic BASELINE scenes use the reference's deterministic lattice (src/mpm.cpp:164-180): the reference's own
     # add_particles(benchmark=125) produces the same positions in the same order as scenes.lattice_block; its benchmark
     # path passes maximum = 1, i.e. vol = dx^3 per particle (an 8x over-dense block) — BASELINE.md keeps the positions
-    # and uses the texture-seeding convention vol = dx^3 / 8 instead
+    # and uses the texture-seeding convention vol = dx^3 / 8 instead.  Stored: the count, a seeded sample of the
+    # positions, and the extremes of the uniform fields.
     res = 40
-    ref = O.ref_benchmark_particles(res, "sand", 125, 400.0)
+    ref = T.live_ref("lattice")
     lo, hi = int(round(res * 0.4)), int(round(res * 0.4)) + int(round(res * 0.2))
     x, mass, vol = scenes.lattice_block(res, (lo,) * 3, (hi,) * 3, 400.0, 0.0)
-    assert len(ref["x"]) == len(x) == 8 ** 3 * 8
-    assert np.abs(ref["x"] - x).max() <= 1.2e-7                      # same lattice, same order (1 ulp)
-    assert np.allclose(ref["vol"], (1.0 / res) ** 3, rtol=1e-6) and np.allclose(vol, (1.0 / res) ** 3 / 8, rtol=1e-6)
-    assert np.allclose(ref["mass"], ref["vol"] * 400.0, rtol=1e-6) and np.allclose(mass, vol * 400.0, rtol=1e-6)
-    assert not ref["v"].any() and np.array_equal(ref["F"], np.tile(np.eye(3, dtype=np.float32).reshape(9), (len(x), 1)))
+    assert int(ref["n"]) == len(x) == 8 ** 3 * 8
+    assert np.abs(ref["x"] - x[ref["ids"]]).max() <= 1.2e-7                # same lattice, same order (1 ulp)
+    assert np.allclose(ref["vol_range"], (1.0 / res) ** 3, rtol=1e-6) and np.allclose(vol, (1.0 / res) ** 3 / 8, rtol=1e-6)
+    assert np.allclose(ref["density_range"], 400.0, rtol=1e-6) and np.allclose(mass, vol * 400.0, rtol=1e-6)
+    assert ref["v_absmax"] == 0 and ref["F_minus_identity_absmax"] == 0
 
 
-@pytest.mark.skipif(not O.ref_transfer_available(), reason="reference tree absent")
 def test_reference_loops_without_particle_gravity_live():
-    # particle_gravity = false: P2G does not touch the particle velocity (src/transfer.cpp:485-487)
-    from tests import common as T
-    scene, st = T.perturbed_scene(scenes.MAT_JELLY, res=24, cells=4, seed=5)
-    scene["particle_gravity"] = 0
-    gv = G.oracle_grid_vel(scene, st)
-    grid, p = O.ref_transfer_substep(scene, st, gv, optimized=True)
-    _compare(scene, st, grid, p)
+    # particle_gravity = false: P2G does not touch the particle velocity (src/transfer.cpp:485-487); the reference's
+    # P2G grid and, for a seeded sample of the particles, its G2P result are stored
+    scene, st = T.no_particle_gravity_scene()
+    r = T.live_ref("no_particle_gravity")
+    nn = tuple(int(v) + 1 for v in scene["res"])
+    grid = np.zeros((int(np.prod(nn)), 4), np.float32)
+    grid[r["grid_idx"]] = r["grid_val"]
+    _compare(scene, st, grid.reshape(nn + (4,)), r, rows=r["ids"])
